@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path (one process per GPU under torchrun)
     python bench.py --impl reference --steps K --warmup W     # the CPU oracle (reference restatement) on the host cores
+    python bench.py --steps K --dump-outputs DIR              # also write the last timed step's poses to DIR/ligand_pos.npy
 
 A "step" is one reverse-diffusion step of the hot path for one batch: set_time -> score-model forward (graph build,
 embeddings, 6 tensor-product conv layers, tr/rot/tor heads) -> pose update, for POSES poses of one synthetic complex
@@ -356,6 +357,21 @@ class Workload:
         return sorted(times)[len(times) // 2], times, final
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(dirname, arrays):
+    """Write each array as DIR/<name>.npy, DUMP_LIMIT_BYTES in all.  An array over its share keeps a fixed, seeded sample of
+    its rows, so the same arguments always select the same rows and two builds stay comparable entry by entry."""
+    os.makedirs(dirname, exist_ok=True)
+    share = DUMP_LIMIT_BYTES // len(arrays)
+    for name, a in arrays.items():
+        if a.nbytes > share:
+            keep = share // (a.nbytes // len(a))
+            a = a[np.sort(np.random.default_rng(0).choice(len(a), keep, replace=False))]
+        np.save(os.path.join(dirname, name + '.npy'), a)
+
+
 def timed_steps(w, steps, warmup_steps, sync_all):
     for i in range(warmup_steps):
         w.step(i)
@@ -371,13 +387,11 @@ def timed_steps(w, steps, warmup_steps, sync_all):
 
 def run_cuda(cli):
     import torch.distributed as dist
-    from diffdock_b200 import ops
-    import __graft_entry__ as ge
+    from diffdock_b200 import ops, _lib
     world = int(os.environ.get('WORLD_SIZE', '1'))
     rank = int(os.environ.get('RANK', '0'))
     local = int(os.environ.get('LOCAL_RANK', '0'))
-    if rank == 0:
-        ge.build()
+    _lib.lib()          # the library build() made; the benchmark compiles nothing
     torch.cuda.set_device(local)
     dev = torch.device('cuda', local)
     if world > 1:
@@ -418,6 +432,10 @@ def run_cuda(cli):
     sync_all()
     ms = e0.elapsed_time(e1) / cli.steps
     clocks = sampler.stop() if sampler else None
+    if cli.dump_outputs and rank == 0:
+        # the ligand coordinates after the last timed step, per pose: what the sampler hands back to its caller
+        pos = w.g['ligand'].pos.detach().float().view(w.n_poses, -1, 3).cpu().numpy()
+        dump_outputs(cli.dump_outputs, {'ligand_pos': pos})
     ms_max = max_over_ranks(ms)
     value = world * cli.poses / (N_SCHED * ms_max * 1e-3)
 
@@ -563,12 +581,11 @@ def run_config5(cli):
     from diffdock_b200.distributed import assign_balanced, sample_complexes_sharded
     from diffdock_b200.sampling import sampling
     from diffdock_b200.synthetic import config5_sizes
-    import __graft_entry__ as ge
+    from diffdock_b200 import _lib
     world = int(os.environ.get('WORLD_SIZE', '1'))
     rank = int(os.environ.get('RANK', '0'))
     local = int(os.environ.get('LOCAL_RANK', '0'))
-    if rank == 0:
-        ge.build()
+    _lib.lib()
     torch.cuda.set_device(local)
     dev = torch.device('cuda', local)
     if world > 1:
@@ -679,7 +696,14 @@ def main():
     ap.add_argument('--quick', action='store_true', help='skip the config-2 / CFG-L1 side measurements')
     ap.add_argument('--short-warmup', dest='short_warmup', action='store_true',
                     help='warm up exactly --warmup steps instead of a full schedule pass (runs under ncu)')
+    ap.add_argument('--dump-outputs', dest='dump_outputs', metavar='DIR',
+                    help='write the ligand coordinates after the last timed step to DIR/ligand_pos.npy (float32, '
+                         '[poses, atoms, 3]); inputs are seeded, so equal arguments give equal inputs')
     cli = ap.parse_args()
+    if cli.steps < 1:
+        ap.error('--steps must be at least 1')
+    if cli.dump_outputs and (cli.impl != 'cuda' or cli.workload != 'single'):
+        ap.error('--dump-outputs applies to the single-complex CUDA workload (--impl cuda --workload single)')
     cli.warmup = max(cli.warmup, 0)
     if cli.impl == 'reference':
         run_reference(cli)
