@@ -21,9 +21,9 @@ from __future__ import annotations
 import torch
 from torch import nn
 
-from . import ops
-from .cg_model import CGModel, _mlp
-from .layers import AtomEncoder
+from . import graphs, ops
+from .cg_model import CGModel
+from .layers import AtomEncoder, _mlp
 from .synthetic import REC_ATOM_FEATURE_DIMS as rec_atom_feature_dims
 from .tensor_layers import TensorProductConvLayer, get_irrep_seq
 
@@ -89,16 +89,10 @@ class AAModel(CGModel):
     def sync_free_capable(self):
         """As CGModel.sync_free_capable; additionally every edge type must have its own radial MLP (the merged single-group
         form concatenates edge lists, which needs their sizes on the host)."""
-        if self._sync_free is None:
-            import os
-            ok = os.environ.get('DDB200_SYNC_FREE', '1') != '0' and self.embed_also_ligand and self.differentiate_convolutions
-            for layer in list(self.conv_layers) + list(self.lig_emb_layers):
-                ok = ok and layer.fused_capable(self.ns, self.ns)
-            self._sync_free = bool(ok)
-        return self._sync_free
+        return self.differentiate_convolutions and super().sync_free_capable()
 
-    def _static(self, data):             # hook of sampling.GraphedSteps: the per-batch constants, outside the capture
-        return self._static_aa(data)
+    def _capacities_fit(self, c):
+        return super()._capacities_fit(c) and c['atom_max'] <= 10000         # the 10000 caps (:595,:610) not binding
 
     # ---------------------------------------------------------------------------------------------------------
     @staticmethod
@@ -107,7 +101,7 @@ class AAModel(CGModel):
         t32, order, _ = ops.csr_sort_by_target(tgt.to(torch.int32).contiguous(), n_rows)
         return (t32, src[order].to(torch.int32).contiguous()) + tuple(p[order].contiguous() for p in payload)
 
-    def _static_aa(self, data):
+    def _static(self, data):
         """Pose-independent part, cached on ``data`` like models/aa_model.py:276-333: residue / atom node embeddings, the
         edge embeddings of the three static graphs (residue-residue, atom-atom, atom-residue), the optional protein
         embedding layers over their four groups, and the CSR-sorted static edge groups of the joint graph."""
@@ -168,33 +162,17 @@ class AAModel(CGModel):
         rr._b200aa = c
         return c
 
-    @torch.no_grad()
-    def forward(self, data):                                            # models/aa_model.py:364-508
-        if self.training:
-            raise RuntimeError("diffdock_b200.AAModel is inference-only: call .eval()")
-        lig, rec, atom = data['ligand'], data['receptor'], data['atom']
-        if not lig.pos.is_cuda:
-            raise RuntimeError("diffdock_b200.AAModel runs on CUDA tensors only (no CPU fallback): data.to('cuda')")
-        if self.no_aminoacid_identities:
-            rec.x = rec.x * 0
-        c = self._static_aa(data)
-        if self.sync_free_capable() and c['rec_max'] <= 10000 and c['atom_max'] <= 10000:     # the 10000 caps (:595,:610) not binding
-            return self._forward_sync_free(data, c)
-        return self._forward_host_sized(data, c)
-
     def _forward_sync_free(self, data, c):
         """The forward without a device->host read (see CGModel._forward_sync_free): ligand graph, ligand-residue and
         ligand-atom graphs written into upper-bound buffers with device-side counts; the reversed groups (residue<-ligand,
         atom<-ligand) are permutations of the forward lists and - as in the reference, models/aa_model.py:405-406 - keep the
         FORWARD direction's edge vector (vec_sign = +1); the four static groups get their sigma term inside the kernel."""
         lig, rec, atom = data['ligand'], data['receptor'], data['atom']
-        ns, B = self.ns, data.num_graphs
-        dev = lig.pos.device
+        ns = self.ns
         tr_sigma, rot_sigma, tor_sigma = self.t_to_sigma(*[data.complex_t[k] for k in ('tr', 'rot', 'tor')])
         n_lig, n_rec = lig.batch.shape[0], rec.batch.shape[0]
         o_r, o_a = n_lig, n_lig + n_rec
         pos, rpos, apos = lig.pos.float().contiguous(), rec.pos.float().contiguous(), atom.pos.float().contiguous()
-        scan = lambda cnt: torch.cumsum(cnt, 0, dtype=torch.int32)
 
         sig = self.rec_sigma_embedding(self.timestep_emb_func(data.complex_t['tr'])).contiguous()
         rec_node, atom_node = rec.rec_node_attr.clone(), atom.atom_node_attr.clone()
@@ -203,54 +181,21 @@ class AAModel(CGModel):
         lig.node_sigma_emb = self.timestep_emb_func(lig.node_t['tr'])
 
         # -- ligand graph: bonds + radius graph (models/aa_model.py:538-568 = cg_model.py:467-497) ---------------------------
-        cnt = ops.radius_count(pos, pos, c['lig_ptr'], c['lig_batch32'], r=self.lig_max_radius, max_num_neighbors=33,
-                               exclude_self=True) + c['pre_cnt']
-        incl = scan(cnt)
-        ll_n = incl[-1:]
-        ll_tgt, ll_src, ll_vec, ll_eid, _ = ops.graph_fill(
-            pos, pos, c['lig_ptr'], c['lig_batch32'], (incl - cnt).contiguous(), c['cap_ll'], r=self.lig_max_radius,
-            max_num_neighbors=33, exclude_self=True, pre_ptr=c['pre_ptr'], pre_col=c['pre_col'], want_eid=True, fill_row=0)
-        ll_attr = torch.cat([c['pre_attr'][ll_eid.long()], lig.node_sigma_emb[ll_tgt.long()],
-                             self.lig_distance_expansion(ll_vec.norm(dim=-1))], 1)
-        ll_ea = self.lig_edge_embedding(ll_attr)
+        g_ll = graphs.ligand_graph(pos, c, self.lig_max_radius, lig.node_sigma_emb, self.lig_distance_expansion,
+                                   self.lig_edge_embedding, self.smooth_edges)
         lig_node = self.lig_node_embedding(torch.cat([lig.x.float(), lig.node_sigma_emb], 1))
-        g_ll = (ll_tgt, ll_src, ll_ea, ll_vec, None, dict(n_edges_dev=ll_n))
         for layer in self.lig_emb_layers:
             lig_node = layer.forward_groups(lig_node, [g_ll], gather_scalars=ns)
 
-        def cross(xpos, x_ptr, x_batch32, x_max, cap, r, rpg, col_off, mlp, gs):
-            """ligand <- x (x = residues or atoms) and its reverse as a permutation; joint numbering offsets applied."""
-            cnt = ops.radius_count(xpos, pos, x_ptr, c['lig_batch32'], r=r, r_per_graph=rpg, max_num_neighbors=10000)
-            incl = scan(cnt)
-            n_dev = incl[-1:]
-            slot = torch.empty((n_lig, max(x_max, 1)), dtype=torch.int32, device=dev)
-            # the embedding kernel only touches live edges; its library fallback gathers over the whole buffer and needs
-            # valid (zero) rows beyond the live count
-            in_kernel = (gs.offset.shape[0], ns) in ops.EDGE_EMBED_SHAPES and len(mlp) == 4
-            f_tgt, f_src, f_vec, _, _ = ops.graph_fill(xpos, pos, x_ptr, c['lig_batch32'], (incl - cnt).contiguous(), cap, r=r,
-                                                       r_per_graph=rpg, max_num_neighbors=10000, slot_out=slot,
-                                                       slot_ld=slot.shape[1], col_offset=col_off,
-                                                       fill_row=None if in_kernel else 0)
-            cnt_r = ops.radius_count(pos, xpos, c['lig_ptr'], x_batch32, r=r, r_per_graph=rpg, max_num_neighbors=1 << 30)
-            incl_r = scan(cnt_r)
-            b_tgt, b_src, _, _, b_perm = ops.graph_fill(pos, xpos, c['lig_ptr'], x_batch32, (incl_r - cnt_r).contiguous(), cap,
-                                                        r=r, r_per_graph=rpg, max_num_neighbors=1 << 30, want_vec=False,
-                                                        slot_in=slot, y_ptr=x_ptr, slot_ld=slot.shape[1], want_perm=True,
-                                                        row_offset=col_off)
-            ea = self._cross_edge_embedding(lig.node_sigma_emb, f_vec, f_tgt, n_dev, mlp=mlp, gs=gs)
-            fwd = (f_tgt, f_src, ea, f_vec, None, dict(n_edges_dev=n_dev))
-            rev = (b_tgt, b_src, ea, f_vec, None, dict(n_edges_dev=n_dev, edge_perm=b_perm, vec_sign=1.0))
-            return fwd, rev
-
         # -- ligand cross graphs (:588-623): residues within the (per-complex) cut-off, atoms within lig_max_radius ---------
-        if self.dynamic_max_cross:
-            rpg, r_cross = (tr_sigma * 3 + 20).reshape(-1).float().contiguous(), 1.0
-        else:
-            rpg, r_cross = None, float(self.cross_max_distance)
-        g_lr, g_rl = cross(rpos, c['rec_ptr'], c['rec_batch32'], c['rec_max'], c['cap_cross'], r_cross, rpg, o_r,
-                           self.lr_edge_embedding, self.cross_distance_expansion)
-        g_la, g_al = cross(apos, c['atom_ptr'], c['atom_batch32'], c['atom_max'], c['cap_la'], float(self.lig_max_radius), None, o_a,
-                           self.la_edge_embedding, self.lig_distance_expansion)
+        r, rpg = graphs.cross_cutoff(tr_sigma, self.dynamic_max_cross, self.cross_max_distance)
+        lr, la = (self.lr_edge_embedding, self.cross_distance_expansion), (self.la_edge_embedding, self.lig_distance_expansion)
+        g_lr, g_rl = graphs.cross_graph(pos, c['lig_ptr'], c['lig_batch32'], rpos, c['rec_ptr'], c['rec_batch32'], c['rec_max'],
+                                        c['cap_cross'], o_r, r, rpg, self._cross_embedder(lig, *lr), vec_sign=1.0,
+                                        fill_row=self._cross_fill_row(*lr))
+        g_la, g_al = graphs.cross_graph(pos, c['lig_ptr'], c['lig_batch32'], apos, c['atom_ptr'], c['atom_batch32'], c['atom_max'],
+                                        c['cap_la'], o_a, float(self.lig_max_radius), None, self._cross_embedder(lig, *la),
+                                        vec_sign=1.0, fill_row=self._cross_fill_row(*la))
 
         # -- joint graph [ligand | residues | atoms]: nine groups in the reference's order (:401-417) --------------------
         node = torch.cat([lig_node, rec_node, atom_node], 0)
@@ -264,11 +209,10 @@ class AAModel(CGModel):
     def _forward_host_sized(self, data, c):
         """Forward with exactly-sized neighbour lists (the sizes are read back to the host)."""
         lig, rec, atom = data['ligand'], data['receptor'], data['atom']
-        ns, B = self.ns, data.num_graphs
+        ns = self.ns
         tr_sigma, rot_sigma, tor_sigma = self.t_to_sigma(*[data.complex_t[k] for k in ('tr', 'rot', 'tor')])
         n_lig, n_rec = lig.pos.shape[0], rec.pos.shape[0]
         o_r, o_a = n_lig, n_lig + n_rec
-        N = o_a + atom.pos.shape[0]
 
         # -- embeddings (:335-362): sigma term on residue / atom scalars and on the three static edge-attribute sets ----
         sig = self.rec_sigma_embedding(self.timestep_emb_func(data.complex_t['tr']))
@@ -285,40 +229,24 @@ class AAModel(CGModel):
             lig_node = layer.forward_groups(lig_node, [g_ll], gather_scalars=ns)
 
         # -- ligand cross graphs (:588-623): residues within the (per-complex) cut-off, atoms within lig_max_radius ---------
-        lp, rp, ap = lig.pos.float(), rec.pos.float(), atom.pos.float()
-        if self.dynamic_max_cross:
-            cutoff = (tr_sigma * 3 + 20).reshape(-1)
-            li, ri, _ = ops.radius(rp, lp, c['rec_ptr'], lig.batch, r=1.0, r_per_graph=cutoff, max_num_neighbors=10000)
-        else:
-            li, ri, _ = ops.radius(rp, lp, c['rec_ptr'], lig.batch, r=float(self.cross_max_distance), max_num_neighbors=10000)
-        li, ri = li.long(), ri.long()
-        lr_vec = rp[ri] - lp[li]
+        lp = lig.pos.float()
+        r, rpg = graphs.cross_cutoff(tr_sigma, self.dynamic_max_cross, self.cross_max_distance)
+        li, ri, lr_vec = graphs.cross_graph_host(lp, rec.pos.float(), c['rec_ptr'], lig.batch, r, rpg)
         lr_ea = self.lr_edge_embedding(torch.cat([lig.node_sigma_emb[li], self.cross_distance_expansion(lr_vec.norm(dim=-1))], 1))
-        la_l, la_a, _ = ops.radius(ap, lp, c['atom_ptr'], lig.batch, r=float(self.lig_max_radius), max_num_neighbors=10000)
-        la_l, la_a = la_l.long(), la_a.long()
-        la_vec = ap[la_a] - lp[la_l]
+        la_l, la_a, la_vec = graphs.cross_graph_host(lp, atom.pos.float(), c['atom_ptr'], lig.batch, float(self.lig_max_radius))
         la_ea = self.la_edge_embedding(torch.cat([lig.node_sigma_emb[la_l], self.lig_distance_expansion(la_vec.norm(dim=-1))], 1))
 
         # -- joint graph [ligand | residues | atoms]: nine groups in the reference's order (:401-417) --------------------
         node = torch.cat([lig_node, rec_node, atom_node], 0)
-        rl_tgt, rl_rev = torch.sort(ri, stable=True)                 # residue <- ligand: same pairs sorted by residue
-        al_tgt, al_rev = torch.sort(la_a, stable=True)               # atom <- ligand
+        g_lr, g_rl = graphs.cross_groups_host(li, ri, o_r, lr_ea, lr_vec, None, vec_sign=1.0)
+        g_la, g_al = graphs.cross_groups_host(la_l, la_a, o_a, la_ea, la_vec, None, vec_sign=1.0)
         stat = lambda k: (c[k][0], c[k][1], c[k][2] + sig[c[k][4]], c[k][3], None)
-        groups = [
-            g_ll,                                                                                        # ligand <- ligand
-            (i32(li), i32(ri + o_r), lr_ea, lr_vec.contiguous(), None),                                  # ligand <- residue
-            (i32(la_l), i32(la_a + o_a), la_ea, la_vec.contiguous(), None),                              # ligand <- atom
-            stat('rr'),                                                                                  # residue <- residue
-            (i32(rl_tgt + o_r), i32(li[rl_rev]), lr_ea[rl_rev], lr_vec[rl_rev].contiguous(), None),      # residue <- ligand (forward Y)
-            stat('ra'),                                                                                  # residue <- atom   (forward Y)
-            stat('aa'),                                                                                  # atom <- atom
-            (i32(al_tgt + o_a), i32(la_l[al_rev]), la_ea[al_rev], la_vec[al_rev].contiguous(), None),    # atom <- ligand    (forward Y)
-            stat('ar'),                                                                                  # atom <- residue
-        ]
+        # reversed groups (residue <- ligand, residue <- atom, atom <- ligand) with the forward harmonics
+        groups = [g_ll, g_lr, g_la, stat('rr'), g_rl, stat('ra'), stat('aa'), g_al, stat('ar')]
         L = len(self.conv_layers)
         for l, layer in enumerate(self.conv_layers):
             use = groups if l < L - 1 else groups[:3]           # last layer: only the groups that end on ligand atoms (:429-430)
             if not self.differentiate_convolutions:             # one radial MLP for all edge types: a single merged group
-                use = [tuple(torch.cat([g[k] for g in use]) if use[0][k] is not None else None for k in range(5))]
+                use = graphs.merge_groups(use)
             node = layer.forward_groups(node, use, gather_scalars=ns)
         return self._heads(data, c, node[:n_lig], tr_sigma, rot_sigma, tor_sigma, sync_free=False)

@@ -18,9 +18,9 @@ import numpy as np
 import torch
 from torch import nn
 
-from . import ops
+from . import graphs, ops
 from .irreps import irreps_str, sh_irreps
-from .layers import AtomEncoder, GaussianSmearing
+from .layers import AtomEncoder, GaussianSmearing, _mlp, edge_weight
 from .synthetic import LIG_FEATURE_DIMS as lig_feature_dims, REC_RESIDUE_FEATURE_DIMS as rec_residue_feature_dims
 from .tensor_layers import TensorProductConvLayer, get_irrep_seq
 from .tp_table import full_tensor_product
@@ -29,10 +29,6 @@ _TABLES = os.path.join(os.path.dirname(os.path.abspath(__file__)), 'tables', 'sc
 # utils/so3.py:6 and utils/torus.py:25-26
 SO3_MIN_EPS, SO3_MAX_EPS, SO3_N_EPS = 0.0005, 4, 2000
 TORUS_SIGMA_MIN, TORUS_SIGMA_MAX, TORUS_SIGMA_N = 3e-3, 2, 5000
-
-
-def _mlp(n_in, n_hidden, n_out, dropout):
-    return nn.Sequential(nn.Linear(n_in, n_hidden), nn.ReLU(), nn.Dropout(dropout), nn.Linear(n_hidden, n_out))
 
 
 def _sh_l2(vec):
@@ -169,12 +165,6 @@ class CGModel(nn.Module):
         self._torus_table.copy_(torch.as_tensor(torus_score_norm, dtype=torch.float32))
 
     # ---------------------------------------------------------------------------------------------------------
-    def get_edge_weight(self, edge_vec, max_norm):
-        if self.smooth_edges:
-            nrm = torch.clip(edge_vec.norm(dim=-1) * np.pi / max_norm, max=np.pi)
-            return 0.5 * (torch.cos(nrm) + 1.0).unsqueeze(-1)
-        return 1.0
-
     def _so3_score_norm(self, eps):
         """utils/so3.py:89-93 evaluated on the device (fp32 index arithmetic, round-half-even like np.around)."""
         lo, hi = math.log10(SO3_MIN_EPS), math.log10(SO3_MAX_EPS)
@@ -208,7 +198,7 @@ class CGModel(nn.Module):
             vec1 = (rec.pos[ei1[1]] - rec.pos[ei1[0]]).float()
             ea1 = self.rec_edge_embedding(self.rec_distance_expansion(vec1.norm(dim=-1)))
             na1 = self.rec_node_embedding(rec.x[:n1])
-            ew1 = self.get_edge_weight(vec1, self.rec_max_radius)
+            ew1 = edge_weight(vec1, self.rec_max_radius, self.smooth_edges)
             for layer in self.rec_emb_layers:
                 ea_ = torch.cat([ea1, na1[ei1[0], :self.ns], na1[ei1[1], :self.ns]], -1)
                 na1 = layer(na1, ei1, ea_, None, edge_weight=ew1, edge_vec=vec1)
@@ -218,7 +208,7 @@ class CGModel(nn.Module):
             vec = (rec.pos[ei[1]] - rec.pos[ei[0]]).float()
             rec_edge_attr = self.rec_edge_embedding(self.rec_distance_expansion(vec.norm(dim=-1)))
             rec_node_attr = self.rec_node_embedding(rec.x)
-            ew = self.get_edge_weight(vec, self.rec_max_radius)
+            ew = edge_weight(vec, self.rec_max_radius, self.smooth_edges)
             for layer in self.rec_emb_layers:
                 ea_ = torch.cat([rec_edge_attr, rec_node_attr[ei[0], :self.ns], rec_node_attr[ei[1], :self.ns]], -1)
                 rec_node_attr = layer(rec_node_attr, ei, ea_, None, edge_weight=ew, edge_vec=vec)
@@ -276,61 +266,46 @@ class CGModel(nn.Module):
 
     def _ligand_graph(self, data, c):
         """Bond edges + radius graph, sorted by convolution target (models/cg_model.py:467-497)."""
-        lig, ll = data['ligand'], data['ligand', 'ligand']
+        lig = data['ligand']
         lig.node_sigma_emb = self.timestep_emb_func(lig.node_t['tr'])
         pos = lig.pos.float()
-        centre, nbr, _ = ops.radius(pos, pos, c['lig_ptr'], lig.batch, r=self.lig_max_radius,
-                                    max_num_neighbors=33, exclude_self=True)      # radius_graph: cap 32 (+ self)
-        n_rad = nbr.shape[0]
-        row0 = torch.cat([ll.edge_index[0].long(), nbr.long()])      # target of the convolution
-        row1 = torch.cat([ll.edge_index[1].long(), centre.long()])   # gathered node
-        bond_attr = torch.cat([ll.edge_attr.float(),
-                               torch.zeros(n_rad, self.in_lig_edge_features, device=pos.device)], 0)
+        row0, row1, bond_attr = graphs.ligand_graph_host(pos, c['lig_ptr'], lig.batch, data['ligand', 'ligand'],
+                                                         self.lig_max_radius, self.in_lig_edge_features)
         tgt, order = torch.sort(row0, stable=True)
         src = row1[order]
         vec = pos[src] - pos[tgt]
         edge_attr = torch.cat([bond_attr[order], lig.node_sigma_emb[tgt], self.lig_distance_expansion(vec.norm(dim=-1))], 1)
         node_attr = torch.cat([lig.x.float(), lig.node_sigma_emb], 1)
-        return node_attr, tgt, src, edge_attr, vec, self.get_edge_weight(vec, self.lig_max_radius)
-
-    def _cross_graph(self, data, c, cutoff):
-        """Ligand-receptor edges within the (per-complex) cutoff, sorted by ligand atom (models/cg_model.py:539-562)."""
-        lig, rec = data['ligand'], data['receptor']
-        lp, rp = lig.pos.float(), rec.pos.float()
-        if torch.is_tensor(cutoff):
-            li, ri, _ = ops.radius(rp, lp, c['rec_ptr'], lig.batch, r=1.0, r_per_graph=cutoff.reshape(-1),
-                                   max_num_neighbors=10000)
-        else:
-            li, ri, _ = ops.radius(rp, lp, c['rec_ptr'], lig.batch, r=float(cutoff), max_num_neighbors=10000)
-        li, ri = li.long(), ri.long()
-        vec = rp[ri] - lp[li]
-        edge_attr = torch.cat([lig.node_sigma_emb[li], self.cross_distance_expansion(vec.norm(dim=-1))], 1)
-        cutoff_d = cutoff.reshape(-1)[lig.batch[li]] if torch.is_tensor(cutoff) else cutoff
-        return li, ri, edge_attr, vec, self.get_edge_weight(vec, cutoff_d)
+        return node_attr, tgt, src, edge_attr, vec, edge_weight(vec, self.lig_max_radius, self.smooth_edges)
 
     # ---------------------------------------------------------------------------------------------------------
     def sync_free_capable(self):
         """The forward can run without any host synchronisation (and so inside a CUDA graph) when every convolution of the
         stack has a shape the fully fused kernel supports; otherwise the neighbour-list sizes go through the host."""
         if self._sync_free is None:
-            ok = os.environ.get('DDB200_SYNC_FREE', '1') != '0'
-            ok = ok and self.embed_also_ligand
+            ok = self.embed_also_ligand
             for layer in list(self.conv_layers) + list(getattr(self, 'lig_emb_layers', [])):
                 ok = ok and layer.fused_capable(self.ns, self.ns)
             self._sync_free = bool(ok)
         return self._sync_free
 
+    def _capacities_fit(self, c):
+        """The 10000-neighbour cap of the cross graph (models/cg_model.py:546) is not binding, so the capacity buffers of the
+        sync-free forward hold every edge."""
+        return c['rec_max'] <= 10000
+
     @torch.no_grad()
     def forward(self, data):
+        name = type(self).__name__
         if self.training:
-            raise RuntimeError("diffdock_b200.CGModel is inference-only: call .eval()")
+            raise RuntimeError(f"diffdock_b200.{name} is inference-only: call .eval()")
         lig, rec = data['ligand'], data['receptor']
         if not lig.pos.is_cuda:
-            raise RuntimeError("diffdock_b200.CGModel runs on CUDA tensors only (no CPU fallback): data.to('cuda')")
+            raise RuntimeError(f"diffdock_b200.{name} runs on CUDA tensors only (no CPU fallback): data.to('cuda')")
         if self.no_aminoacid_identities:
             rec.x = rec.x * 0
         c = self._static(data)
-        if self.sync_free_capable() and c['rec_max'] <= 10000:      # cap of the cross graph (models/cg_model.py:546) not binding
+        if self.sync_free_capable() and self._capacities_fit(c):
             return self._forward_sync_free(data, c)
         return self._forward_host_sized(data, c)
 
@@ -342,12 +317,10 @@ class CGModel(nn.Module):
         take (capacity, device count).  Shapes are static for a given batch, so a reverse-diffusion step can be captured in
         a CUDA graph (diffdock_b200/sampling.py)."""
         lig, rec = data['ligand'], data['receptor']
-        ns, B = self.ns, data.num_graphs
-        dev = lig.pos.device
+        ns = self.ns
         tr_sigma, rot_sigma, tor_sigma = self.t_to_sigma(*[data.complex_t[k] for k in ('tr', 'rot', 'tor')])
-        n_lig, n_rec = lig.batch.shape[0], rec.batch.shape[0]
+        n_lig = lig.batch.shape[0]
         pos, rpos = lig.pos.float().contiguous(), rec.pos.float().contiguous()
-        scan = lambda cnt: torch.cumsum(cnt, 0, dtype=torch.int32)
 
         # -- embeddings (models/cg_model.py:272-306) --------------------------------------------------------------
         sig = self.rec_sigma_embedding(self.timestep_emb_func(data.complex_t['tr'])).contiguous()      # [B, ns]
@@ -356,53 +329,18 @@ class CGModel(nn.Module):
         lig.node_sigma_emb = self.timestep_emb_func(lig.node_t['tr'])
 
         # -- ligand graph: bonds + radius graph, CSR by target, built on the device (:467-497) -------------------------
-        cnt = ops.radius_count(pos, pos, c['lig_ptr'], c['lig_batch32'], r=self.lig_max_radius, max_num_neighbors=33,
-                               exclude_self=True) + c['pre_cnt']
-        incl = scan(cnt)
-        ll_n = incl[-1:]
-        ll_tgt, ll_src, ll_vec, ll_eid, _ = ops.graph_fill(
-            pos, pos, c['lig_ptr'], c['lig_batch32'], (incl - cnt).contiguous(), c['cap_ll'], r=self.lig_max_radius,
-            max_num_neighbors=33, exclude_self=True, pre_ptr=c['pre_ptr'], pre_col=c['pre_col'], want_eid=True, fill_row=0)
-        tgt_l = ll_tgt.long()
-        ll_attr = torch.cat([c['pre_attr'][ll_eid.long()], lig.node_sigma_emb[tgt_l],
-                             self.lig_distance_expansion(ll_vec.norm(dim=-1))], 1)
-        ll_ea = self.lig_edge_embedding(ll_attr)
-        ll_ew = self.get_edge_weight(ll_vec, self.lig_max_radius)
+        g_ll = graphs.ligand_graph(pos, c, self.lig_max_radius, lig.node_sigma_emb, self.lig_distance_expansion,
+                                   self.lig_edge_embedding, self.smooth_edges)
         lig_node = self.lig_node_embedding(torch.cat([lig.x.float(), lig.node_sigma_emb], 1))
-        ewt = lambda w: w.reshape(-1).contiguous() if torch.is_tensor(w) else None
-        g_ll = (ll_tgt, ll_src, ll_ea, ll_vec, ewt(ll_ew), dict(n_edges_dev=ll_n))
         for layer in self.lig_emb_layers:
             lig_node = layer.forward_groups(lig_node, [g_ll], gather_scalars=ns)
 
         # -- cross graph, both directions (:321-327, :539-562) ------------------------------------------------------------
-        if self.dynamic_max_cross:
-            rpg, r_cross = (tr_sigma * 3 + 20).reshape(-1).float().contiguous(), 1.0
-        else:
-            rpg, r_cross = None, float(self.cross_max_distance)
-        cap = c['cap_cross']
-        cnt = ops.radius_count(rpos, pos, c['rec_ptr'], c['lig_batch32'], r=r_cross, r_per_graph=rpg, max_num_neighbors=10000)
-        incl = scan(cnt)
-        lr_n = incl[-1:]
-        slot = torch.empty((n_lig, max(c['rec_max'], 1)), dtype=torch.int32, device=dev)
-        # rows beyond the live count must be valid (zero) when library ops gather over the whole buffer: the smooth edge
-        # weight, or the embedding MLP when its shape is outside the edge-embedding kernel's templates
-        smooth = self.smooth_edges or not ((self.cross_distance_expansion.offset.shape[0], ns) in ops.EDGE_EMBED_SHAPES
-                                           and len(self.cross_edge_embedding) == 4)
-        lr_tgt, lr_src, lr_vec, _, _ = ops.graph_fill(
-            rpos, pos, c['rec_ptr'], c['lig_batch32'], (incl - cnt).contiguous(), cap, r=r_cross, r_per_graph=rpg,
-            max_num_neighbors=10000, slot_out=slot, slot_ld=slot.shape[1], col_offset=n_lig, fill_row=0 if smooth else None)
-        cnt_r = ops.radius_count(pos, rpos, c['lig_ptr'], c['rec_batch32'], r=r_cross, r_per_graph=rpg,
-                                 max_num_neighbors=1 << 30)
-        incl_r = scan(cnt_r)
-        rl_tgt, rl_src, _, _, rl_perm = ops.graph_fill(
-            pos, rpos, c['lig_ptr'], c['rec_batch32'], (incl_r - cnt_r).contiguous(), cap, r=r_cross, r_per_graph=rpg,
-            max_num_neighbors=1 << 30, want_vec=False, slot_in=slot, y_ptr=c['rec_ptr'], slot_ld=slot.shape[1],
-            want_perm=True, row_offset=n_lig)
-        lr_ea = self._cross_edge_embedding(lig.node_sigma_emb, lr_vec, lr_tgt, lr_n)
-        lr_ew = None
-        if self.smooth_edges:
-            cutoff_d = rpg[lig.batch[lr_tgt.long()]] if rpg is not None else r_cross
-            lr_ew = ewt(self.get_edge_weight(lr_vec, cutoff_d))
+        r, rpg = graphs.cross_cutoff(tr_sigma, self.dynamic_max_cross, self.cross_max_distance)
+        lr = (self.cross_edge_embedding, self.cross_distance_expansion)
+        g_lr, g_rl = graphs.cross_graph(pos, c['lig_ptr'], c['lig_batch32'], rpos, c['rec_ptr'], c['rec_batch32'], c['rec_max'],
+                                        c['cap_cross'], n_lig, r, rpg, self._cross_embedder(lig, *lr, r, rpg), vec_sign=-1.0,
+                                        fill_row=self._cross_fill_row(*lr))
 
         # -- joint graph: four edge groups (:329-338) ---------------------------------------------------------------
         node = torch.cat([lig_node, rec_node], 0)
@@ -412,10 +350,10 @@ class CGModel(nn.Module):
             rr_tgt32 = c['rr_tgt32'][n_lig] = (i32(c['rr_tgt'] + n_lig), i32(c['rr_src'] + n_lig))
         groups = [
             g_ll,                                                                                         # lig <- lig
-            (lr_tgt, lr_src, lr_ea, lr_vec, lr_ew, dict(n_edges_dev=lr_n)),                               # lig <- rec
-            (rr_tgt32[0], rr_tgt32[1], c['rr_ea'], c['rr_vec'], ewt(c['rr_ew']),
+            g_lr,                                                                                         # lig <- rec
+            (rr_tgt32[0], rr_tgt32[1], c['rr_ea'], c['rr_vec'], graphs.flat_weight(c['rr_ew']),
              dict(ea_add=sig, ea_add_idx=c['rr_gid32'])),                                                 # rec <- rec
-            (rl_tgt, rl_src, lr_ea, lr_vec, lr_ew, dict(n_edges_dev=lr_n, edge_perm=rl_perm, vec_sign=-1.0)),   # rec <- lig
+            g_rl,                                                                                         # rec <- lig
         ]
         L = len(self.conv_layers)
         shared = self._shared_receptor_messages(data, c, rec, rec_node, sig, n_lig) if L > 1 else None
@@ -456,27 +394,44 @@ class CGModel(nn.Module):
         cnt_buf[n_lig:].view(B, n1).add_(cnt0.unsqueeze(0))
         return sum_buf, cnt_buf
 
-    def _cross_edge_embedding(self, node_sigma_emb, vec, row, n_dev, mlp=None, gs=None):
-        """cross_edge_embedding(cat[sigma_emb[lig], RBF(d)]) (models/cg_model.py:326,553-554): the sigma half of the first
-        Linear is applied per ligand NODE, the rest per edge in one kernel (ddb200_edge_embed).  ``mlp`` / ``gs``: another
-        embedding MLP / distance expansion of the same form (the all-atom model's ligand-residue and ligand-atom edges)."""
-        mlp = self.cross_edge_embedding if mlp is None else mlp
-        gs = self.cross_distance_expansion if gs is None else gs
+    def _cross_edge_embedding(self, node_sigma_emb, vec, row, n_dev, mlp, gs):
+        """``mlp``(cat[sigma_emb[lig], ``gs``(d)]) of ligand <- x edges, e.g. cross_edge_embedding with the cross distance
+        expansion (models/cg_model.py:326,553-554): the sigma half of the first Linear is applied per ligand NODE, the rest
+        per edge in one kernel (ddb200_edge_embed)."""
         l1, l2 = mlp[0], mlp[-1]
         S = node_sigma_emb.shape[1]
-        if (gs.offset.shape[0], self.ns) in ops.EDGE_EMBED_SHAPES and len(mlp) == 4:
+        if self._edge_embed_in_kernel(mlp, gs):
             u = torch.addmm(l1.bias, node_sigma_emb, l1.weight[:, :S].t()).contiguous()
             return ops.edge_embed(vec, row, u, l1.weight[:, S:].contiguous(), l2.weight.contiguous(), l2.bias.contiguous(),
                                   gs.offset.contiguous(), float(gs.coeff), n_dev)
         attr = torch.cat([node_sigma_emb[row.long()], gs(vec.norm(dim=-1))], 1)      # library path on the padded buffer
         return mlp(attr)
 
+    def _cross_embedder(self, lig, mlp, gs, r=None, rpg=None):
+        """``embed`` of graphs.cross_graph: edge attributes through ``mlp`` / ``gs`` and, with smooth_edges, the edge weight
+        at the cut-off (``r``, or ``rpg`` per complex)."""
+        def embed(tgt, vec, n_dev):
+            ea = self._cross_edge_embedding(lig.node_sigma_emb, vec, tgt, n_dev, mlp, gs)
+            if not self.smooth_edges:
+                return ea, None
+            return ea, graphs.flat_weight(edge_weight(vec, rpg[lig.batch[tgt.long()]] if rpg is not None else r, True))
+        return embed
+
+    def _edge_embed_in_kernel(self, mlp, gs):
+        return (gs.offset.shape[0], self.ns) in ops.EDGE_EMBED_SHAPES and len(mlp) == 4
+
+    def _cross_fill_row(self, mlp, gs):
+        """``fill_row`` of a sync-free cross graph: rows beyond the live count must be valid (zero) when library ops gather
+        over the whole buffer - the smooth edge weight, or the embedding MLP when its shape is outside the edge-embedding
+        kernel's templates."""
+        return 0 if self.smooth_edges or not self._edge_embed_in_kernel(mlp, gs) else None
+
     # ---------------------------------------------------------------------------------------------------------
     def _forward_host_sized(self, data, c):
         """Forward with exactly-sized neighbour lists (one host read of each edge count): convolution shapes outside the
         fused kernel's templates, or more than 10000 residues per complex."""
         lig, rec = data['ligand'], data['receptor']
-        ns, B = self.ns, data.num_graphs
+        ns = self.ns
         tr_sigma, rot_sigma, tor_sigma = self.t_to_sigma(*[data.complex_t[k] for k in ('tr', 'rot', 'tor')])
 
         # -- embeddings (models/cg_model.py:272-306) --------------------------------------------------------------
@@ -494,31 +449,33 @@ class CGModel(nn.Module):
             lig_node = layer(lig_node, ll_ei, ea_, None, edge_weight=ll_ew, edge_vec=ll_vec, assume_sorted=True)
 
         # -- cross graph (:321-327) ---------------------------------------------------------------------------------
-        cutoff = (tr_sigma * 3 + 20).unsqueeze(1) if self.dynamic_max_cross else self.cross_max_distance
-        li, ri, lr_ea, lr_vec, lr_ew = self._cross_graph(data, c, cutoff)
+        lp = lig.pos.float()
+        r, rpg = graphs.cross_cutoff(tr_sigma, self.dynamic_max_cross, self.cross_max_distance)
+        li, ri, lr_vec = graphs.cross_graph_host(lp, rec.pos.float(), c['rec_ptr'], lig.batch, r, rpg)
+        lr_ea = torch.cat([lig.node_sigma_emb[li], self.cross_distance_expansion(lr_vec.norm(dim=-1))], 1)
+        cutoff_d = rpg[lig.batch[li]] if rpg is not None else r
+        lr_ew = edge_weight(lr_vec, cutoff_d, self.smooth_edges)
         lr_ea = self.cross_edge_embedding(lr_ea)
 
         # -- joint graph: four edge groups, each CSR-sorted by target (:329-338) ------------------------------------
         n_lig = lig_node.shape[0]
         node = torch.cat([lig_node, rec_node], 0)
-        rl_tgt, rev = torch.sort(ri, stable=True)            # receptor <- ligand direction: same pairs, sorted by residue
         i32 = lambda t: t.to(torch.int32).contiguous()
-        ewt = lambda w: w.reshape(-1).contiguous() if torch.is_tensor(w) else None
         rr_tgt32 = c.setdefault('rr_tgt32', {}).get(n_lig)
         if rr_tgt32 is None:      # static receptor graph: int32 indices in the joint numbering, once per batch
             rr_tgt32 = c['rr_tgt32'][n_lig] = (i32(c['rr_tgt'] + n_lig), i32(c['rr_src'] + n_lig))
+        g_lr, g_rl = graphs.cross_groups_host(li, ri, n_lig, lr_ea, lr_vec, lr_ew, vec_sign=-1.0)
         groups = [   # (target, gathered node, edge attr, edge vector, edge weight): int32, CSR-sorted, built once per forward
-            (i32(ll_tgt), i32(ll_src), ll_ea, ll_vec.contiguous(), ewt(ll_ew)),                          # lig <- lig
-            (i32(li), i32(ri + n_lig), lr_ea, lr_vec.contiguous(), ewt(lr_ew)),                          # lig <- rec
-            (rr_tgt32[0], rr_tgt32[1], rr_ea, c['rr_vec'], ewt(c['rr_ew'])),                             # rec <- rec
-            (i32(rl_tgt + n_lig), i32(li[rev]), lr_ea[rev], (-lr_vec[rev]).contiguous(),
-             ewt(lr_ew[rev]) if torch.is_tensor(lr_ew) else None),                                       # rec <- lig, SH(-v)
+            (i32(ll_tgt), i32(ll_src), ll_ea, ll_vec.contiguous(), graphs.flat_weight(ll_ew)),           # lig <- lig
+            g_lr,                                                                                        # lig <- rec
+            (rr_tgt32[0], rr_tgt32[1], rr_ea, c['rr_vec'], graphs.flat_weight(c['rr_ew'])),              # rec <- rec
+            g_rl,                                                                                        # rec <- lig, SH(-v)
         ]
         L = len(self.conv_layers)
         for l, layer in enumerate(self.conv_layers):
             use = groups if l < L - 1 else groups[:2]       # last layer: only edges that end on ligand atoms (:347-349)
             if not self.differentiate_convolutions:         # one radial MLP for all edge types: a single merged group
-                use = [tuple(torch.cat([g[k] for g in use]) if use[0][k] is not None else None for k in range(5))]
+                use = graphs.merge_groups(use)
             node = layer.forward_groups(node, use, gather_scalars=ns)
         lig_node = node[:n_lig]
         return self._heads(data, c, lig_node, tr_sigma, rot_sigma, tor_sigma, sync_free=False)
@@ -560,11 +517,9 @@ class CGModel(nn.Module):
         if sync_free:
             # upper-bound buffer (32 atoms per bond, models/cg_model.py:630); slots beyond the live count point at an extra
             # dummy bond row (index n_bonds) that is dropped after the convolution
-            pos_c = pos.contiguous()
-            cnt = ops.radius_count(pos_c, bond_pos, c['lig_ptr'], c['bond_batch32'], r=self.lig_max_radius, max_num_neighbors=32)
-            incl = torch.cumsum(cnt, 0, dtype=torch.int32)
-            bi32, ai32, t_vec, _, _ = ops.graph_fill(pos_c, bond_pos, c['lig_ptr'], c['bond_batch32'], (incl - cnt).contiguous(),
-                                                     c['cap_tor'], r=self.lig_max_radius, max_num_neighbors=32, fill_row=n_bonds)
+            bi32, ai32, t_vec, _, _, _ = graphs.capacity_graph(pos.contiguous(), bond_pos, c['lig_ptr'], c['bond_batch32'],
+                                                               c['cap_tor'], self.lig_max_radius, max_num_neighbors=32,
+                                                               fill_row=n_bonds)
             bi, ai = bi32.long(), ai32.long()
             bi_g = bi.clamp_max(n_bonds - 1)            # gathers of per-bond quantities for the dummy slots: any valid row
             n_out = n_bonds + 1
@@ -579,7 +534,7 @@ class CGModel(nn.Module):
         t_sh = torch.einsum('ea,eb,abc->ec', _sh_full(t_vec, self.sh_lmax), _sh_l2(bond_vec)[bi_g], self._tor_tp)
         t_ea = torch.cat([t_ea, lig_node[ai, :ns], bond_attr[bi_g, :ns]], -1)
         tor_pred = self.tor_bond_conv(lig_node, torch.stack([bi, ai]), t_ea, t_sh, out_nodes=n_out, reduce='mean',
-                                      edge_weight=self.get_edge_weight(t_vec, self.lig_max_radius), assume_sorted=True)
+                                      edge_weight=edge_weight(t_vec, self.lig_max_radius, self.smooth_edges), assume_sorted=True)
         tor_pred = self.tor_final_layer(tor_pred[:n_bonds]).squeeze(1)
         edge_sigma = tor_sigma[c['bond_lig_batch']]
         if self.scale_by_sigma:

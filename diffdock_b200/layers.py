@@ -1,9 +1,24 @@
 """Embedding layers with the reference's parameter names (models/layers.py) - plain PyTorch modules on the device
 (small dense ops; the hot convolution lives in csrc/)."""
+import numpy as np
 import torch
 from torch import nn
 
 from .tensor_layers import FCBlock  # noqa: F401  (re-export: the reference keeps FCBlock in models/layers.py)
+
+
+def _mlp(n_in, n_hidden, n_out, dropout):
+    """Linear - ReLU - Dropout - Linear: the edge / sigma embeddings of the models."""
+    return nn.Sequential(nn.Linear(n_in, n_hidden), nn.ReLU(), nn.Dropout(dropout), nn.Linear(n_hidden, n_out))
+
+
+def edge_weight(edge_vec, max_norm, smooth):
+    """Edge weight of smooth_edges, 0.5 (cos(pi |v| / max_norm) + 1) clipped at |v| = max_norm, else the constant 1
+    (models/cg_model.py:459-465).  ``max_norm`` is a number or a per-edge tensor."""
+    if smooth:
+        nrm = torch.clip(edge_vec.norm(dim=-1) * np.pi / max_norm, max=np.pi)
+        return 0.5 * (torch.cos(nrm) + 1.0).unsqueeze(-1)
+    return 1.0
 
 
 class GaussianSmearing(nn.Module):

@@ -15,24 +15,20 @@ CUDA only, inference only.  No CPU fallback.
 """
 from __future__ import annotations
 
-import numpy as np
 import torch
 import torch.nn.functional as F
 from torch import nn
 
-from . import ops
+from . import graphs, ops
 from .irreps import irreps_str, sh_irreps
-from .layers import GaussianSmearing, OldAtomEncoder
+from .layers import GaussianSmearing, OldAtomEncoder, _mlp, edge_weight
+from .old_cg_model import ConfidenceModel
 from .synthetic import (LIG_FEATURE_DIMS as lig_feature_dims, REC_ATOM_FEATURE_DIMS as rec_atom_feature_dims,
                         REC_RESIDUE_FEATURE_DIMS as rec_residue_feature_dims)
 from .tensor_layers import OldTensorProductConvLayer
 
 
-def _mlp(n_in, n_hidden, n_out, dropout):
-    return nn.Sequential(nn.Linear(n_in, n_hidden), nn.ReLU(), nn.Dropout(dropout), nn.Linear(n_hidden, n_out))
-
-
-class AAOldModel(nn.Module):
+class AAOldModel(ConfidenceModel):
     def __init__(self, t_to_sigma, device, timestep_emb_func, in_lig_edge_features=4, sigma_embed_dim=32, sh_lmax=2,
                  ns=16, nv=4, num_conv_layers=2, lig_max_radius=5, rec_max_radius=30, cross_max_distance=250,
                  center_max_distance=30, distance_embed_dim=32, cross_distance_embed_dim=32, no_torsion=False,
@@ -92,17 +88,6 @@ class AAOldModel(nn.Module):
             nn.Linear(2 * ns if num_conv_layers >= 3 else ns, ns), bn(), nn.ReLU(), nn.Dropout(confidence_dropout),
             nn.Linear(ns, ns), bn(), nn.ReLU(), nn.Dropout(confidence_dropout), nn.Linear(ns, out_dim))
 
-    def load_state_dict(self, state_dict, strict=True, **kw):
-        """Reference checkpoints carry e3nn's tensor-product buffers (``*.tp.*``): dropped, the kernels have their own tables."""
-        sd = {k: v for k, v in state_dict.items() if '.tp.' not in k}
-        return super().load_state_dict(sd, strict=strict, **kw)
-
-    def get_edge_weight(self, edge_vec, max_norm):                      # models/old_aa_model.py:352-356
-        if self.smooth_edges:
-            nn_ = torch.clip(edge_vec.norm(dim=-1) * np.pi / max_norm, max=np.pi)
-            return 0.5 * (torch.cos(nn_) + 1.0).unsqueeze(-1)
-        return 1.0
-
     def _static_graph(self, data, nt, pos, edge_embedding, node_embedding, expansion, max_r):
         """Receptor-residue / receptor-atom graph on precomputed edges (:400-445); row 0 = target, row 1 = gathered node."""
         st = data[nt]
@@ -111,7 +96,7 @@ class AAOldModel(nn.Module):
         vec = pos[ei[1]] - pos[ei[0]]
         ea = edge_embedding(torch.cat([st.node_sigma_emb[ei[0]], expansion(vec.norm(dim=-1))], 1))
         node = node_embedding(torch.cat([st.x.float(), st.node_sigma_emb], 1))
-        return node, ei, ea, vec, self.get_edge_weight(vec, max_r)
+        return node, ei, ea, vec, edge_weight(vec, max_r, self.smooth_edges)
 
     @torch.no_grad()
     def forward(self, data):                                            # models/old_aa_model.py:202-286
@@ -130,15 +115,12 @@ class AAOldModel(nn.Module):
 
         # ligand graph (:358-398): bonds + radius graph
         lig_s.node_sigma_emb = self.timestep_emb_func(lig_s.node_t['tr'])
-        ll = data['ligand', 'ligand']
-        centre, nbr, _ = ops.radius(lp, lp, lig_ptr, lig_s.batch, r=self.lig_max_radius, max_num_neighbors=33,
-                                    exclude_self=True)                  # radius_graph: cap 32 (+ self)
-        lig_ei = torch.stack([torch.cat([ll.edge_index[0].long(), nbr.long()]),
-                              torch.cat([ll.edge_index[1].long(), centre.long()])])
+        row0, row1, bond_attr = graphs.ligand_graph_host(lp, lig_ptr, lig_s.batch, data['ligand', 'ligand'],
+                                                         self.lig_max_radius, self.in_lig_edge_features)
+        lig_ei = torch.stack([row0, row1])
         lig_vec = lp[lig_ei[1]] - lp[lig_ei[0]]
-        lig_ea = torch.cat([torch.cat([ll.edge_attr.float(), lp.new_zeros(nbr.shape[0], self.in_lig_edge_features)], 0),
-                            lig_s.node_sigma_emb[lig_ei[0]], self.lig_distance_expansion(lig_vec.norm(dim=-1))], 1)
-        lig_w = self.get_edge_weight(lig_vec, self.lig_max_radius)
+        lig_ea = torch.cat([bond_attr, lig_s.node_sigma_emb[lig_ei[0]], self.lig_distance_expansion(lig_vec.norm(dim=-1))], 1)
+        lig_w = edge_weight(lig_vec, self.lig_max_radius, self.smooth_edges)
         lig = self.lig_node_embedding(torch.cat([lig_s.x.float(), lig_s.node_sigma_emb], 1))
         lig_ea = self.lig_edge_embedding(lig_ea)
 
@@ -150,23 +132,17 @@ class AAOldModel(nn.Module):
                                                               self.lig_max_radius)
 
         # cross graphs (:447-491): ligand-residue (cut-off per complex), ligand-atom (lig_max_radius), atom-residue (given)
-        if self.dynamic_max_cross:
-            cutoff = (tr_sigma * 3 + 20).reshape(-1)
-            li, ri, _ = ops.radius(rp, lp, rec_ptr, lig_s.batch, r=1.0, r_per_graph=cutoff, max_num_neighbors=10000)
-        else:
-            cutoff = self.cross_max_distance
-            li, ri, _ = ops.radius(rp, lp, rec_ptr, lig_s.batch, r=float(cutoff), max_num_neighbors=10000)
-        lr = torch.stack([li.long(), ri.long()])
-        lr_vec = rp[lr[1]] - lp[lr[0]]
+        r, rpg = graphs.cross_cutoff(tr_sigma, self.dynamic_max_cross, self.cross_max_distance)
+        li, ri, lr_vec = graphs.cross_graph_host(lp, rp, rec_ptr, lig_s.batch, r, rpg)
+        lr = torch.stack([li, ri])
         lr_ea = self.lr_edge_embedding(torch.cat([lig_s.node_sigma_emb[lr[0]],
                                                   self.cross_distance_expansion(lr_vec.norm(dim=-1))], 1))
-        lr_w = self.get_edge_weight(lr_vec, cutoff[lig_s.batch[lr[0]]] if torch.is_tensor(cutoff) else cutoff)
-        la_l, la_a, _ = ops.radius(ap, lp, atom_ptr, lig_s.batch, r=float(self.lig_max_radius), max_num_neighbors=10000)
-        la = torch.stack([la_l.long(), la_a.long()])
-        la_vec = ap[la[1]] - lp[la[0]]
+        lr_w = edge_weight(lr_vec, rpg[lig_s.batch[lr[0]]] if rpg is not None else r, self.smooth_edges)
+        la_l, la_a, la_vec = graphs.cross_graph_host(lp, ap, atom_ptr, lig_s.batch, float(self.lig_max_radius))
+        la = torch.stack([la_l, la_a])
         la_ea = self.la_edge_embedding(torch.cat([lig_s.node_sigma_emb[la[0]],
                                                   self.cross_distance_expansion(la_vec.norm(dim=-1))], 1))
-        la_w = self.get_edge_weight(la_vec, self.lig_max_radius)
+        la_w = edge_weight(la_vec, self.lig_max_radius, self.smooth_edges)
         ar = data['atom', 'receptor'].edge_index.long()
         ar_vec = rp[ar[1]] - ap[ar[0]]
         ar_ea = self.ar_edge_embedding(torch.cat([atom_s.node_sigma_emb[ar[0]],
@@ -197,7 +173,4 @@ class AAOldModel(nn.Module):
             if l != L - 1:
                 atom = F.pad(atom, (0, at_up.shape[-1] - atom.shape[-1])) + at_up + al_up + ar_up
                 rec = F.pad(rec, (0, rec_up.shape[-1] - rec.shape[-1])) + rec_up + ra_up + rl_up
-        scal = torch.cat([lig[:, :ns], lig[:, -ns:]], 1) if L >= 3 else lig[:, :ns]
-        pooled = torch.zeros((B, scal.shape[1]), device=scal.device, dtype=scal.dtype).index_add_(0, lig_s.batch, scal)
-        pooled = pooled / torch.bincount(lig_s.batch, minlength=B).clamp(min=1).unsqueeze(1)
-        return self.confidence_predictor(pooled).squeeze(dim=-1)
+        return self._confidence(lig, lig_s.batch, B)

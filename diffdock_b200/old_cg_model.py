@@ -12,23 +12,37 @@ CUDA only, inference only.  No CPU fallback.
 """
 from __future__ import annotations
 
-import numpy as np
 import torch
 import torch.nn.functional as F
 from torch import nn
 
-from . import ops
+from . import graphs, ops
 from .irreps import irreps_str, sh_irreps
-from .layers import GaussianSmearing, OldAtomEncoder
+from .layers import GaussianSmearing, OldAtomEncoder, _mlp, edge_weight
 from .synthetic import LIG_FEATURE_DIMS as lig_feature_dims, REC_RESIDUE_FEATURE_DIMS as rec_residue_feature_dims
 from .tensor_layers import OldTensorProductConvLayer
 
 
-def _mlp(n_in, n_hidden, n_out, dropout):
-    return nn.Sequential(nn.Linear(n_in, n_hidden), nn.ReLU(), nn.Dropout(dropout), nn.Linear(n_hidden, n_out))
+class ConfidenceModel(nn.Module):
+    """What the coarse-grained and the all-atom confidence models share: loading reference checkpoints, and the head that
+    pools the ligand's scalar features per complex."""
+
+    def load_state_dict(self, state_dict, strict=True, **kw):
+        """Reference checkpoints carry e3nn's tensor-product buffers (``*.tp.*``): dropped, the kernels have their own tables."""
+        sd = {k: v for k, v in state_dict.items() if '.tp.' not in k}
+        return super().load_state_dict(sd, strict=strict, **kw)
+
+    def _confidence(self, lig_node, lig_batch, B):
+        """confidence_predictor of the per-complex mean of the ligand scalars: the 0e channels, and the 0o channels too with
+        three or more layers (models/old_cg_model.py:285-301)."""
+        ns = self.ns
+        scal = torch.cat([lig_node[:, :ns], lig_node[:, -ns:]], 1) if self.num_conv_layers >= 3 else lig_node[:, :ns]
+        pooled = torch.zeros((B, scal.shape[1]), device=scal.device, dtype=scal.dtype).index_add_(0, lig_batch, scal)
+        pooled = pooled / torch.bincount(lig_batch, minlength=B).clamp(min=1).unsqueeze(1)
+        return self.confidence_predictor(pooled).squeeze(dim=-1)
 
 
-class CGOldModel(nn.Module):
+class CGOldModel(ConfidenceModel):
     def __init__(self, t_to_sigma, device, timestep_emb_func, in_lig_edge_features=4, sigma_embed_dim=32, sh_lmax=2,
                  ns=16, nv=4, num_conv_layers=2, lig_max_radius=5, rec_max_radius=30, cross_max_distance=250,
                  center_max_distance=30, distance_embed_dim=32, cross_distance_embed_dim=32, no_torsion=False,
@@ -87,17 +101,6 @@ class CGOldModel(nn.Module):
             nn.Linear(ns, ns), bn(), nn.ReLU(), nn.Dropout(confidence_dropout),
             nn.Linear(ns, 2 if affinity_prediction else 1))
 
-    def load_state_dict(self, state_dict, strict=True, **kw):
-        """Reference checkpoints carry e3nn's tensor-product buffers (``*.tp.*``): dropped, the kernels have their own tables."""
-        sd = {k: v for k, v in state_dict.items() if '.tp.' not in k}
-        return super().load_state_dict(sd, strict=strict, **kw)
-
-    def get_edge_weight(self, edge_vec, max_norm):                      # models/old_cg_model.py:353-359
-        if self.smooth_edges:
-            nn_ = torch.clip(edge_vec.norm(dim=-1) * np.pi / max_norm, max=np.pi)
-            return 0.5 * (torch.cos(nn_) + 1.0).unsqueeze(-1)
-        return 1.0
-
     @torch.no_grad()
     def forward(self, data):                                            # models/old_cg_model.py:203-301
         if self.training:
@@ -114,15 +117,12 @@ class CGOldModel(nn.Module):
 
         # ligand graph (:361-391): bonds + radius graph; row 0 = convolution target, row 1 = gathered node
         lig.node_sigma_emb = self.timestep_emb_func(lig.node_t['tr'])
-        ll = data['ligand', 'ligand']
-        centre, nbr, _ = ops.radius(lp, lp, lig_ptr, lig.batch, r=self.lig_max_radius, max_num_neighbors=33,
-                                    exclude_self=True)                  # radius_graph: cap 32 (+ self)
-        lig_ei = torch.stack([torch.cat([ll.edge_index[0].long(), nbr.long()]),
-                              torch.cat([ll.edge_index[1].long(), centre.long()])])
+        row0, row1, bond_attr = graphs.ligand_graph_host(lp, lig_ptr, lig.batch, data['ligand', 'ligand'], self.lig_max_radius,
+                                                         self.in_lig_edge_features)
+        lig_ei = torch.stack([row0, row1])
         lig_vec = lp[lig_ei[1]] - lp[lig_ei[0]]
-        lig_ea = torch.cat([torch.cat([ll.edge_attr.float(), lp.new_zeros(nbr.shape[0], self.in_lig_edge_features)], 0),
-                            lig.node_sigma_emb[lig_ei[0]], self.lig_distance_expansion(lig_vec.norm(dim=-1))], 1)
-        lig_ew = self.get_edge_weight(lig_vec, self.lig_max_radius)
+        lig_ea = torch.cat([bond_attr, lig.node_sigma_emb[lig_ei[0]], self.lig_distance_expansion(lig_vec.norm(dim=-1))], 1)
+        lig_ew = edge_weight(lig_vec, self.lig_max_radius, self.smooth_edges)
         lig_node = self.lig_node_embedding(torch.cat([lig.x.float(), lig.node_sigma_emb], 1))
         lig_ea = self.lig_edge_embedding(lig_ea)
 
@@ -132,22 +132,16 @@ class CGOldModel(nn.Module):
         rec_vec = rp[rec_ei[1]] - rp[rec_ei[0]]
         rec_ea = self.rec_edge_embedding(torch.cat([rec.node_sigma_emb[rec_ei[0]],
                                                     self.rec_distance_expansion(rec_vec.norm(dim=-1))], 1))
-        rec_ew = self.get_edge_weight(rec_vec, self.rec_max_radius)
+        rec_ew = edge_weight(rec_vec, self.rec_max_radius, self.smooth_edges)
         rec_node = self.rec_node_embedding(torch.cat([rec.x.float(), rec.node_sigma_emb], 1))
 
         # cross graph (:439-461): row 0 = ligand atom, row 1 = receptor residue, vector receptor - ligand
-        if self.dynamic_max_cross:
-            cutoff = (tr_sigma * 3 + 20).reshape(-1)
-            li, ri, _ = ops.radius(rp, lp, rec_ptr, lig.batch, r=1.0, r_per_graph=cutoff, max_num_neighbors=10000)
-        else:
-            cutoff = self.cross_max_distance
-            li, ri, _ = ops.radius(rp, lp, rec_ptr, lig.batch, r=float(cutoff), max_num_neighbors=10000)
-        li, ri = li.long(), ri.long()
+        r, rpg = graphs.cross_cutoff(tr_sigma, self.dynamic_max_cross, self.cross_max_distance)
+        li, ri, lr_vec = graphs.cross_graph_host(lp, rp, rec_ptr, lig.batch, r, rpg)
         lr_ei, rl_ei = torch.stack([li, ri]), torch.stack([ri, li])
-        lr_vec = rp[ri] - lp[li]
         lr_ea = self.cross_edge_embedding(torch.cat([lig.node_sigma_emb[li],
                                                      self.cross_distance_expansion(lr_vec.norm(dim=-1))], 1))
-        lr_ew = self.get_edge_weight(lr_vec, cutoff[lig.batch[li]] if torch.is_tensor(cutoff) else cutoff)
+        lr_ew = edge_weight(lr_vec, rpg[lig.batch[li]] if rpg is not None else r, self.smooth_edges)
 
         L = len(self.lig_conv_layers)
         for l in range(L):
@@ -166,7 +160,4 @@ class CGOldModel(nn.Module):
             lig_node = F.pad(lig_node, (0, lig_intra.shape[-1] - lig_node.shape[-1])) + lig_intra + lig_inter
             if l != L - 1:
                 rec_node = F.pad(rec_node, (0, rec_intra.shape[-1] - rec_node.shape[-1])) + rec_intra + rec_inter
-        scal = torch.cat([lig_node[:, :ns], lig_node[:, -ns:]], 1) if self.num_conv_layers >= 3 else lig_node[:, :ns]
-        pooled = torch.zeros((B, scal.shape[1]), device=scal.device, dtype=scal.dtype).index_add_(0, lig.batch, scal)
-        pooled = pooled / torch.bincount(lig.batch, minlength=B).clamp(min=1).unsqueeze(1)
-        return self.confidence_predictor(pooled).squeeze(dim=-1)
+        return self._confidence(lig_node, lig.batch, B)
